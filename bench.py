@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — tokens/s of the data-parallel pretraining step (forward + backward + sharded AdamW) on synthetic tokens.
 
-    python bench.py --gpus N --steps K --warmup W [--workload NAME] [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--workload NAME] [--impl reference] [--dump-outputs DIR]
 
 Workloads (BASELINE.json `configs`):
     gpt2-110m        C2  Wenzhong-GPT2-110M, seq 1024, 32 sequences per GPU, bf16            (default at any N; weak scaling)
@@ -25,6 +25,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.join(ROOT, "fengshen-lm_b200"))
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 import torch.distributed as dist  # noqa: E402
 
@@ -353,10 +354,29 @@ def cpu_reference_run(w, steps, warmup, budget_s=None):
             "sample": sample, "cores": n_thr}
 
 
-def run_workload(name, args, world, rank, device, pg, steps, warmup, want_e2e=True, profile_steps=2, overrides=None):
+DUMP_PARAMS = 8 << 20   # parameter elements written by --dump-outputs (32 MB as float32)
+
+
+def dump_outputs(out_dir, loss, stepper):
+    """What the timed step hands its caller: the step's mean loss and the updated parameters. Models larger than DUMP_PARAMS
+    elements are sampled at fixed positions (seed 0), so two builds run with the same arguments write comparable files."""
+    stepper.engine.wait_params()
+    params = stepper.model.flat.params
+    n = params.numel()
+    if n > DUMP_PARAMS:
+        idx = torch.randint(0, n, (DUMP_PARAMS,), generator=torch.Generator().manual_seed(0)).sort().values
+        params = params[idx.to(params.device)]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "loss.npy"), loss.detach().float().cpu().numpy())
+    np.save(os.path.join(out_dir, "params.npy"), params.float().cpu().numpy())
+
+
+def run_workload(name, args, world, rank, device, pg, steps, warmup, want_e2e=True, profile_steps=2, overrides=None,
+                 dump_dir=None):
     """Build the model + engine for workload `name`, warm up, time `steps` optimizer steps with the batches resident in
     HBM (`value`), then through the public API from pinned host memory (`e2e`), then `profile_steps` EXTRA steps with CUDA
-    events around every GEMM launch (the roofline block) — the timed regions themselves carry no instrumentation."""
+    events around every GEMM launch (the roofline block) — the timed regions themselves carry no instrumentation.
+    With `dump_dir`, rank 0 writes the outputs of the last `value` step there before any further step runs."""
     from fsb200 import lib as L, ops
     from fsb200.schedules import polynomial_lr
     from fsb200.trainer import PretrainStep
@@ -386,6 +406,8 @@ def run_workload(name, args, world, rank, device, pg, steps, warmup, want_e2e=Tr
     ms = timed(lambda i: losses.append(stepper.step_device(dev[i % pool])), steps, world)
     clocks = sampler.stop() if sampler else None
     launches = L.kernel_launches - k0
+    if dump_dir and rank == 0:
+        dump_outputs(dump_dir, losses[-1], stepper)
     ms_per_step = ms / steps
     value = world * tokens_step_gpu / (ms_per_step / 1000.0)
 
@@ -545,7 +567,14 @@ def main():
     ap.add_argument("--breakdown", action="store_true",
                     help="after the timed runs, profile 2 more steps with CUDA events around every fsb_* call and print the "
                          "per-entry-point time table to stderr (diagnostic; not part of the JSON line)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last step's loss and updated parameters (a fixed sample of at most "
+                         f"{DUMP_PARAMS} elements) as float32 DIR/loss.npy and DIR/params.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs records the fsb200 step; the reference arm has nothing to write")
     w = workload(args.workload)
     over = {}
     if args.micro_batch:
@@ -594,7 +623,7 @@ def main():
 
     warm = max(3, args.warmup)
     main_run = run_workload(args.workload, args, world, rank, device, pg, args.steps, warm, want_e2e=not args.no_e2e,
-                            overrides=over)
+                            overrides=over, dump_dir=args.dump_outputs)
     graph_block = None
     if world == 1 and not args.cuda_graph and not args.no_graph_block:
         # the same workload with the whole optimizer step captured in ONE CUDA graph and replayed (bit-identical results,

@@ -1,7 +1,11 @@
 """TEST INFRASTRUCTURE — seeded inputs for the Megatron index builders (`helpers`: build_sample_idx, build_mapping,
 build_blocks_mapping, build_blending_indices). `run_cases(helpers_module)` runs them against ANY implementation with the
 reference's call signatures: oracle/make_golden_index_builders.py feeds it the reference's own C++ compiled into oracle/_ref/
-(-> tests/golden/index_builders.npz), tests/test_index_builders_cpu.py feeds it the fsb200 compat module and compares."""
+(-> tests/golden/index_builders.npz), tests/test_index_builders_cpu.py feeds it the fsb200 compat module and compares.
+`random_cases` does the same on randomised inputs; its reference outputs are kept as digests
+(oracle/make_golden_reference_runs.py -> tests/golden/index_builders_random.json)."""
+import hashlib
+
 import numpy as np
 
 
@@ -53,4 +57,42 @@ def run_cases(H):
         ds = np.zeros(size, dtype=np.int64)
         H.build_blending_indices(di, ds, np.asarray(w, dtype=np.float64), len(w), size, False)
         out[f"blend_index_{i}"], out[f"blend_sample_{i}"] = di, ds
+    return out
+
+
+def digest(a):
+    """SHA-256 of an array's dtype, shape and bytes: exact equality at a fraction of the array's size."""
+    a = np.ascontiguousarray(a)
+    return hashlib.sha256(f"{a.dtype.str}{a.shape}".encode() + a.tobytes()).hexdigest()
+
+
+def random_cases(H, trials=40):
+    """Randomised corpora and arguments (seed 31337), every builder per trial: `{trial}_mapping`, `_blocks`, `_sample_idx`,
+    `_blend_index`, `_blend_sample`."""
+    out = {}
+    rs = np.random.RandomState(31337)
+    for trial in range(trials):
+        n_docs = int(rs.randint(1, 400))
+        docs, sizes = corpus(rs, n_docs, max_sent=int(rs.randint(1, 15)), max_len=int(rs.randint(2, 200)),
+                             p_empty=rs.rand() * 0.3, p_long=rs.rand() * 0.05)
+        titles = rs.randint(0, 30, size=n_docs).astype(np.int32)
+        epochs, seed = int(rs.randint(1, 5)), int(rs.randint(1, 2 ** 31 - 1))
+        cap = int(rs.choice([10 ** 9, rs.randint(1, 200)]))
+        max_len = int(rs.randint(8, 600))
+        p_short = float(rs.choice([0.0, 0.1, 0.33, 1.0]))
+        min_sent = int(rs.randint(1, 4))
+        one = bool(rs.randint(0, 2))
+        out[f"{trial}_mapping"] = np.asarray(H.build_mapping(docs, sizes, epochs, cap, max_len, p_short, seed, False, min_sent))
+        out[f"{trial}_blocks"] = np.asarray(H.build_blocks_mapping(docs, sizes, titles, epochs, cap, max_len, seed, False, one))
+        tok = rs.randint(0, 60, size=n_docs).astype(np.int32)
+        seq = int(rs.randint(2, 100))
+        tok[rs.randint(0, n_docs)] += seq + 1
+        order = np.concatenate([rs.permutation(n_docs) for _ in range(epochs)]).astype(np.int32)
+        out[f"{trial}_sample_idx"] = np.asarray(H.build_sample_idx(tok, order, seq, epochs, int(tok.sum())))
+        nd = int(rs.randint(1, 12))
+        w = rs.dirichlet(np.ones(nd))
+        size = int(rs.randint(0, 3000))
+        a, b = np.zeros(size, np.uint8), np.zeros(size, np.int64)
+        H.build_blending_indices(a, b, w, nd, size, False)
+        out[f"{trial}_blend_index"], out[f"{trial}_blend_sample"] = a, b
     return out

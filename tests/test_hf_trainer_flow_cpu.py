@@ -94,11 +94,14 @@ def _rank_main(rank, world, port, workdir, q):
     torch.distributed.destroy_process_group()
 
 
-def test_erlangshen_recipe_two_ranks_over_gloo(tmp_path):
+def test_erlangshen_recipe_two_ranks_over_gloo(tmp_path, monkeypatch):
     import json
     import numpy as np
     import torch
     import torch.multiprocessing as mp
+    # the ranks inherit this: they take the host path (gloo, CPU kernels) on machines with a GPU too, where the compat Trainer
+    # would otherwise bind rank r to cuda:r over NCCL
+    monkeypatch.setenv("CUDA_VISIBLE_DEVICES", "")
     F.bert_dir(tmp_path / "m")
     F.bert_corpus(tmp_path / "train.json", n=64)
     (tmp_path / "ds_config.json").write_text(json.dumps({"zero_optimization": {"stage": 1}, "bf16": {"enabled": True},
